@@ -90,6 +90,9 @@ def parse():
     ap.add_argument("--height", type=int, default=H45)
     ap.add_argument("--e2e-steps", type=int, default=12)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the C3 chain returned in its last step to DIR/c3_out.npy (float32 RGBA; the whole "
+                         "frame when it fits 64 MB, else a fixed seeded sample of its pixels in ascending order)")
     ap.add_argument("--no-batch", action="store_true", help="skip the 64-frame batch export (BASELINE.json configs[4])")
     ap.add_argument("--c4", action="store_true", help="at N > 1: also the 100 MP C4 chain over the ranks (always run at N = 4, the configuration BASELINE.json names)")
     ap.add_argument("--no-other-modules", action="store_true", help="skip the untimed per-module table of the non-C2 modules")
@@ -97,6 +100,23 @@ def parse():
                     help="internal: run the pipe-end module table in this process and print it as one JSON object (the main run calls this in a "
                          "child process so that code which has not been through a GPU round cannot take the headline down)")
     return ap.parse_args()
+
+
+DUMP_BYTES = 64_000_000
+DUMP_PIXELS = 1 << 21          # 32 MiB of RGBA float32
+
+
+def dump_outputs(out_dir, frame):
+    """write the (h, w, 4) device frame to out_dir/c3_out.npy: whole, or DUMP_PIXELS-odd pixels drawn with the bench seed"""
+    os.makedirs(out_dir, exist_ok=True)
+    px = frame.reshape(-1, 4)
+    if px.numel() * 4 <= DUMP_BYTES:
+        arr = frame.cpu().numpy()
+    else:
+        import torch
+        idx = np.unique(np.random.default_rng(SEED).integers(0, px.shape[0], DUMP_PIXELS))
+        arr = px[torch.from_numpy(idx).to(px.device)].cpu().numpy()
+    np.save(os.path.join(out_dir, "c3_out.npy"), np.ascontiguousarray(arr, np.float32))
 
 
 def peaks():
@@ -662,6 +682,8 @@ def run_b200(args):
     L.b200_kernel_timing(1)
     with ClockSampler(local) as clk:
         ms_max, mod_ms = timed_steps(c3, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, c3.out)
     ksum, kcnt = C.c_double(), C.c_int()
     kernel_ms = {}
     for name in ("nlm_kernel", "rcd_tiles_kernel"):

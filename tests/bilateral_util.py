@@ -61,6 +61,7 @@ def emul_bilateral(img, ss, sr, detail, grid_after=None):
     return _run(emul_lib(), "emul_bilateral", img, ss, sr, detail, grid_after)
 
 
+@util.recorded(lambda img, ss, sr, detail, threads=1, kind="strict": oracle_bilateral(img, ss, sr, detail)[1])
 def ref_bilateral(img, ss, sr, detail, threads=1, kind="strict"):
     lib = util.ref(kind)
     if lib is None:
@@ -76,6 +77,7 @@ def ref_bilateral(img, ss, sr, detail, threads=1, kind="strict"):
     return np.array(out)
 
 
+@util.recorded(lambda img, ss, sr, blur, threads=1, kind="strict": oracle_bilateral(img, ss, sr, 0.0, "blur" if blur else "splat")[2:])
 def ref_grid(img, ss, sr, blur, threads=1, kind="strict"):
     lib = util.ref(kind)
     h, w = img.shape[:2]

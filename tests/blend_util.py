@@ -124,6 +124,7 @@ def oracle(a, b, p, form=None, xoffs=0, yoffs=0):
     return _run(util.oracle(), "orc_blend_process", a, b, p, form, xoffs, yoffs)
 
 
+@util.recorded(lambda a, b, p, form=None, xoffs=0, yoffs=0, kind="strict": oracle(a, b, p, form, xoffs, yoffs))
 def ref(a, b, p, form=None, xoffs=0, yoffs=0, kind="strict"):
     lib = util.ref(kind)
     fn = {CS_LAB: "ref_blend_lab_process", CS_RGB_DISPLAY: "ref_blend_rgb_hsl_process", CS_RAW: "ref_blend_raw_process"}.get(p.blend_cst, "ref_blend_process")

@@ -61,10 +61,15 @@ def _call(f, img, filters, clips, iterations, scales, noise_level, solid_color, 
     return out, np.array(list(nv), np.float32)
 
 
+@util.recorded(lambda img, filters, clips, *, iterations=2, scales=6, noise_level=0.0, solid_color=0.0, iscale=1.0, roi_scale=1.0, norm=None, x=0, y=0,
+               xtrans=None, lib=None, threads=None: oracle(img, filters, clips, iterations=iterations, scales=scales, noise_level=noise_level,
+                                                           solid_color=solid_color, iscale=iscale, roi_scale=roi_scale, norm=norm, x=x, y=y, xtrans=xtrans))
 def ref(img, filters, clips, *, iterations=2, scales=6, noise_level=0.0, solid_color=0.0, iscale=1.0, roi_scale=1.0, norm=None, x=0, y=0,
-        xtrans=None, lib=None):
-    """the reference's process_laplacian(); returns (output, the normalization vector the run used)"""
+        xtrans=None, lib=None, threads=None):
+    """the reference's process_laplacian(); returns (output, the normalization vector the run used); threads: OpenMP threads"""
     lib = lib or util.ref("strict")
+    if threads:
+        C.CDLL("libgomp.so.1").omp_set_num_threads(threads)
     return _call(lib.ref_hl_laplacian, img, filters, clips, iterations, scales, noise_level, solid_color, iscale, roi_scale, norm,
                  norm is not None, x, y, xtrans)
 

@@ -36,6 +36,7 @@ def oracle(m, filters, mode, carry=0):
     return _run(util.oracle(), "orc_lmmse", m, filters, mode, (carry,))
 
 
+@util.recorded(lambda m, filters, mode, kind="strict": oracle(m, filters, mode, carry=1))
 def ref(m, filters, mode, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _run(lib, "ref_lmmse", m, filters, mode)

@@ -37,6 +37,7 @@ def oracle(m, x=0, y=0, passes=1):
     return _call(util.oracle(), "orc_markesteijn", m, x, y, passes)
 
 
+@util.recorded(lambda m, x=0, y=0, passes=1, kind="strict": oracle(m, x, y, passes))
 def ref(m, x=0, y=0, passes=1, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _call(lib, "ref_markesteijn", m, x, y, passes)

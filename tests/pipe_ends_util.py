@@ -50,6 +50,7 @@ def oracle_rawprepare(piece, src: np.ndarray) -> np.ndarray:
     return out
 
 
+@util.recorded(lambda piece, src, gain=None, spacing=(0.0, 0.0), origin=(0.0, 0.0), kind="strict": oracle_rawprepare(piece, src))
 def ref_rawprepare(piece, src: np.ndarray, gain=None, spacing=(0.0, 0.0), origin=(0.0, 0.0), kind="strict"):
     lib = util.ref(kind)
     if lib is None:
@@ -97,6 +98,7 @@ def oracle_temperature(piece, img: np.ndarray) -> np.ndarray:
     return out
 
 
+@util.recorded(lambda piece, img, kind="strict": oracle_temperature(piece, img))
 def ref_temperature(piece, img: np.ndarray, kind="strict"):
     lib = util.ref(kind)
     if lib is None:
@@ -123,6 +125,7 @@ def oracle_highlights(piece, img: np.ndarray):
     return rc, out, n.value
 
 
+@util.recorded(lambda piece, img, kind="strict": oracle_highlights(piece, img)[1])
 def ref_highlights(piece, img: np.ndarray, kind="strict"):
     lib = util.ref(kind)
     if lib is None:
@@ -149,6 +152,7 @@ def oracle_exposure(piece, img: np.ndarray) -> np.ndarray:
     return out
 
 
+@util.recorded(lambda piece, img, kind="strict": oracle_exposure(piece, img))
 def ref_exposure(piece, img: np.ndarray, kind="strict"):
     lib = util.ref(kind)
     if lib is None:
@@ -170,6 +174,7 @@ def oracle_gamma(img: np.ndarray, fill: int = 0x5A) -> np.ndarray:
     return out
 
 
+@util.recorded(lambda img, fill=0x5A, kind="strict": oracle_gamma(img, fill))
 def ref_gamma(img: np.ndarray, fill: int = 0x5A, kind="strict"):
     lib = util.ref(kind)
     if lib is None:
@@ -193,6 +198,7 @@ def oracle_export(img: np.ndarray, fmt: int) -> np.ndarray:
     return out
 
 
+@util.recorded(lambda img, fmt, kind="strict": oracle_export(img, fmt))
 def ref_export(img: np.ndarray, fmt: int, kind="strict"):
     lib = util.ref(kind)
     if lib is None:
@@ -234,6 +240,7 @@ def oracle_plan(*a):
     return _plan(util.oracle(), "orc_resampling_plan", *a)
 
 
+@util.recorded(lambda *a, kind="strict": oracle_plan(*a))
 def ref_plan(*a, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _plan(lib, "ref_resampling_plan", *a)
@@ -255,6 +262,7 @@ def oracle_finalscale(img, out_w, out_h, in_scale, out_scale, interpolator):
     return _finalscale(util.oracle(), "orc_finalscale", img, out_w, out_h, in_scale, out_scale, interpolator)
 
 
+@util.recorded(lambda img, out_w, out_h, in_scale, out_scale, interpolator, kind="strict": oracle_finalscale(img, out_w, out_h, in_scale, out_scale, interpolator))
 def ref_finalscale(img, out_w, out_h, in_scale, out_scale, interpolator, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _finalscale(lib, "ref_finalscale", img, out_w, out_h, in_scale, out_scale, interpolator)
@@ -270,6 +278,7 @@ def oracle_channelmixerrgb(img, cp):
     return out
 
 
+@util.recorded(lambda img, cp, kind="strict": oracle_channelmixerrgb(img, cp))
 def ref_channelmixerrgb(img, cp, kind="strict"):
     lib = util.ref(kind)
     if lib is None:
@@ -301,6 +310,7 @@ def oracle_clip_and_zoom(img, roi_in, roi_out, interpolator):
     return _clip_and_zoom(util.oracle(), "orc_clip_and_zoom", img, roi_in, roi_out, interpolator)
 
 
+@util.recorded(lambda img, roi_in, roi_out, interpolator, kind="strict": oracle_clip_and_zoom(img, roi_in, roi_out, interpolator))
 def ref_clip_and_zoom(img, roi_in, roi_out, interpolator, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _clip_and_zoom(lib, "ref_clip_and_zoom", img, roi_in, roi_out, interpolator)
@@ -323,6 +333,7 @@ def oracle_flip(img, orientation):
     return _flip(util.oracle(), "orc_flip", img, orientation, "bpp")
 
 
+@util.recorded(lambda img, orientation, kind="strict": oracle_flip(img, orientation))
 def ref_flip(img, orientation, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _flip(lib, "ref_flip", img, orientation, "bpp")

@@ -46,6 +46,7 @@ def oracle_ppg(mosaic, filters, thrs=0.0):
     return _run(util.oracle(), "orc_demosaic_ppg", mosaic, filters, thrs)
 
 
+@util.recorded(lambda mosaic, filters, thrs=0.0, kind="strict": oracle_ppg(mosaic, filters, thrs))
 def ref_ppg(mosaic, filters, thrs=0.0, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _run(lib, "ref_demosaic_ppg", mosaic, filters, thrs)
@@ -83,6 +84,7 @@ def oracle_passthrough(m, filters, x=0, y=0, colour=0):
     return _passthrough(util.oracle(), "orc_demosaic_passthrough", m, filters, x, y, colour)
 
 
+@util.recorded(lambda m, filters, x=0, y=0, colour=0, kind="strict": oracle_passthrough(m, filters, x, y, colour))
 def ref_passthrough(m, filters, x=0, y=0, colour=0, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _passthrough(lib, "ref_demosaic_passthrough", m, filters, x, y, colour)
@@ -108,6 +110,7 @@ def oracle_downsample(m, filters):
     return _downsample(util.oracle(), "orc_demosaic_downsample", m, filters)
 
 
+@util.recorded(lambda m, filters, kind="strict": oracle_downsample(m, filters))
 def ref_downsample(m, filters, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _downsample(lib, "ref_demosaic_downsample", m, filters)
@@ -134,6 +137,7 @@ def oracle_downsample_xtrans(m, x, y, xtrans):
     return _downsample_xtrans(util.oracle(), "orc_demosaic_downsample_xtrans", m, x, y, xtrans)
 
 
+@util.recorded(lambda m, x, y, xtrans, kind="strict": oracle_downsample_xtrans(m, x, y, xtrans))
 def ref_downsample_xtrans(m, x, y, xtrans, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _downsample_xtrans(lib, "ref_demosaic_downsample_xtrans", m, x, y, xtrans)
@@ -159,6 +163,7 @@ def oracle_postfilter(rgba, iterations):
     return _postfilter(util.oracle(), "orc_demosaic_downsample_postfilter", rgba, iterations)
 
 
+@util.recorded(lambda rgba, iterations, kind="strict": oracle_postfilter(rgba, iterations))
 def ref_postfilter(rgba, iterations, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _postfilter(lib, "ref_demosaic_downsample_postfilter", rgba, iterations)
@@ -188,6 +193,7 @@ def oracle_downsample4(m, filters, cam_to_rgb=CYGM_TO_RGB):
     return _downsample4(util.oracle(), "orc_demosaic_downsample4", m, filters, cam_to_rgb)
 
 
+@util.recorded(lambda m, filters, cam_to_rgb=CYGM_TO_RGB, kind="strict": oracle_downsample4(m, filters, cam_to_rgb))
 def ref_downsample4(m, filters, cam_to_rgb=CYGM_TO_RGB, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _downsample4(lib, "ref_demosaic_downsample4", m, filters, cam_to_rgb)

@@ -22,10 +22,8 @@ def _build():
         util.build_oracle()
 
 
-need_ref = pytest.mark.skipif(util.ref("strict") is None and not os.path.isdir("/root/reference/src"), reason="oracle/_ref not built (no /root/reference)")
 
 
-@need_ref
 @pytest.mark.parametrize("name", list(bu.CASES))
 def test_bilateral_oracle_equals_one_slice_reference(name):
     img, ss, sr, detail = bu.case(name)
@@ -36,7 +34,6 @@ def test_bilateral_oracle_equals_one_slice_reference(name):
     assert same_bits(bu.oracle_bilateral(img, ss, sr, detail, "blur")[3], bu.ref_grid(img, ss, sr, blur=1, threads=1)[1]).all()
 
 
-@need_ref
 def test_reference_splat_depends_on_the_thread_count():
     """the partial grids of the slices are added after the fact: cells fed by two slices round differently"""
     img, ss, sr, detail = bu.case("coarse_smoothing")

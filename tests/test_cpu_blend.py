@@ -22,11 +22,9 @@ def _build():
         util.build_oracle()
 
 
-need_ref = pytest.mark.skipif(util.ref("strict") is None and not os.path.isdir("/root/reference/src"), reason="oracle/_ref not built (no /root/reference)")
 IDS = [c[0] for c in bu.CONFIGS]
 
 
-@need_ref
 @pytest.mark.parametrize("cfg", bu.CONFIGS, ids=IDS)
 def test_oracle_equals_reference(cfg):
     name, kw, uses_form = cfg
@@ -39,7 +37,6 @@ def test_oracle_equals_reference(cfg):
     assert (name == "disabled") == np.array_equal(out_r, b)      # every other configuration changes the output
 
 
-@need_ref
 def test_oracle_equals_reference_with_roi_out_inside_roi_in():
     a, b, form = bu.frames(100, 80, 2, xoffs=7, yoffs=5)
     for name, kw, uses_form in bu.CONFIGS[::3]:
@@ -74,7 +71,6 @@ def test_kernel_with_offsets_and_what_is_refused():
 LAB_IDS = [c[0] for c in bu.LAB_CONFIGS]
 
 
-@need_ref
 @pytest.mark.parametrize("cfg", bu.LAB_CONFIGS, ids=LAB_IDS)
 def test_lab_oracle_equals_reference(cfg):
     """every operator of the Lab space, the L / a / b / C / h channels of the parametric mask, the other mask sources"""
@@ -88,7 +84,6 @@ def test_lab_oracle_equals_reference(cfg):
     assert not np.array_equal(out_r[..., :3], b[..., :3])
 
 
-@need_ref
 def test_lab_oracle_equals_reference_with_roi_out_inside_roi_in():
     a, b, form = bu.frames_lab(100, 80, 2, xoffs=7, yoffs=5)
     for name, kw, uses_form in bu.LAB_CONFIGS[::4]:
@@ -128,7 +123,6 @@ def test_oracle_and_kernel_against_the_committed_reference_output(cfg):
 DISPLAY_IDS = [c[0] for c in bu.DISPLAY_CONFIGS]
 
 
-@need_ref
 @pytest.mark.parametrize("cfg", bu.DISPLAY_CONFIGS, ids=DISPLAY_IDS)
 def test_display_oracle_equals_reference(cfg):
     """every operator of the display-referred space, the gray / R / G / B / H / S / L channels of the parametric mask, the other mask sources"""
@@ -153,7 +147,6 @@ def test_display_kernel_equals_oracle(cfg):
 
 
 # ---- the raw space (develop/blends/blendif_raw.c): one float per site ------------------------------------------------------------------------
-@need_ref
 @pytest.mark.parametrize("cfg", bu.RAW_CONFIGS, ids=[c[0] for c in bu.RAW_CONFIGS])
 def test_raw_reference_oracle_and_kernel(cfg):
     name, kw, uses_form = cfg
@@ -217,7 +210,6 @@ def random_parameter_block(rng):
     return cst, kw, uses_form
 
 
-@need_ref
 def test_random_parameter_blocks_reference_oracle_and_kernel_agree():
     """the four colour spaces"""
     rng = np.random.default_rng(123)

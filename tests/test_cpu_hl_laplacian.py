@@ -24,8 +24,6 @@ CASES = [
 
 @pytest.mark.parametrize("name,w,h,filters,kw", CASES, ids=[c[0] for c in CASES])
 def test_oracle_is_the_reference(name, w, h, filters, kw):
-    if util.ref("strict") is None:
-        pytest.skip("oracle/_ref not built")
     m = hu.clipped_mosaic(w, h, len(name))
     want, norm = hu.ref(m, filters, hu.clips_of(), **kw)
     got, _ = hu.oracle(m, filters, hu.clips_of(), norm=norm, **kw)
@@ -35,8 +33,6 @@ def test_oracle_is_the_reference(name, w, h, filters, kw):
 
 
 def test_oracle_is_the_reference_on_rgba_input():
-    if util.ref("strict") is None:
-        pytest.skip("oracle/_ref not built")
     img = hu.clipped_rgba(300, 200, 4)
     want, norm = hu.ref(img, 0, hu.clips_of(), iterations=2, noise_level=0.1)
     got, _ = hu.oracle(img, 0, hu.clips_of(), norm=norm, iterations=2, noise_level=0.1)
@@ -49,8 +45,6 @@ XCASES = [("xtrans", 300, 200, dict(xtrans=hu.XTRANS)), ("xtrans_roi_noise", 251
 
 @pytest.mark.parametrize("name,w,h,kw", XCASES, ids=[c[0] for c in XCASES])
 def test_oracle_is_the_reference_on_xtrans(name, w, h, kw):
-    if util.ref("strict") is None:
-        pytest.skip("oracle/_ref not built")
     m = hu.clipped_mosaic(w, h, 3)
     want, norm = hu.ref(m, 9, hu.clips_of(), **kw)
     got, _ = hu.oracle(m, 9, hu.clips_of(), norm=norm, **kw)
@@ -67,18 +61,11 @@ def test_kernels_thread_by_thread_xtrans(name, w, h, kw):
 def test_normalization_is_the_serial_sum_of_one_thread():
     """the reference's vector is an OpenMP float reduction: with one thread it is the oracle's row-order sum, bit for bit, and with many it is
     another value; the frames agree closely all the same (the vector divides the gathered frame and multiplies the result back)"""
-    if util.ref("strict") is None:
-        pytest.skip("oracle/_ref not built")
-    omp = C.CDLL("libgomp.so.1")
     m = hu.clipped_mosaic(640, 480, 11)
-    omp.omp_set_num_threads(1)
-    try:
-        want, norm1 = hu.ref(m, RGGB, hu.clips_of())
-    finally:
-        omp.omp_set_num_threads(8)
+    want, norm1 = hu.ref(m, RGGB, hu.clips_of(), threads=1)
     got, norm_o = hu.oracle(m, RGGB, hu.clips_of())
     assert same_bits(norm1, norm_o).all() and same_bits(got, want).all()
-    many, norm8 = hu.ref(m, RGGB, hu.clips_of())
+    many, norm8 = hu.ref(m, RGGB, hu.clips_of(), threads=8)
     exact = np.array([m[0::2, 0::2].sum(dtype=np.float64), m[0::2, 1::2].sum(dtype=np.float64) + m[1::2, 0::2].sum(dtype=np.float64),
                       m[1::2, 1::2].sum(dtype=np.float64)]) / m.size
     assert np.abs(norm8[:3] / exact - 1).max() < 1e-4 and np.abs(norm1[:3] / exact - 1).max() < 1e-3
@@ -125,8 +112,6 @@ def test_oracle_against_the_committed_reference_output(name):
 
 def test_random_frames_and_parameters_reference_oracle_and_kernels_agree():
     """frames from 8 px a side, the three layouts, ROI origins, zoom, the scale parameter from 0, noise and solid colour, clip levels"""
-    if util.ref("strict") is None:
-        pytest.skip("oracle/_ref not built")
     rng = np.random.default_rng(7)
     for trial in range(40):
         w, h, kind = int(rng.integers(8, 180)), int(rng.integers(8, 140)), int(rng.integers(3))

@@ -23,10 +23,8 @@ def _build():
         util.build_oracle()
 
 
-need_ref = pytest.mark.skipif(util.ref("strict") is None and not os.path.isdir("/root/reference/src"), reason="oracle/_ref not built (no /root/reference)")
 
 
-@need_ref
 @pytest.mark.parametrize("mode", [0, 1, 2, 3, 4])
 @pytest.mark.parametrize("name", list(lu.CASES))
 def test_oracle_with_carried_planes_equals_reference(name, mode):

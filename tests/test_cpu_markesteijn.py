@@ -24,10 +24,8 @@ def _build():
         util.build_oracle()
 
 
-need_ref = pytest.mark.skipif(util.ref("strict") is None and not os.path.isdir("/root/reference/src"), reason="oracle/_ref not built (no /root/reference)")
 
 
-@need_ref
 @pytest.mark.parametrize("passes", [1, 3])
 @pytest.mark.parametrize("name", list(mu.CASES))
 def test_oracle_equals_reference(name, passes):
@@ -48,7 +46,6 @@ def test_oracle_equals_golden(name):
             assert same_bits(mu.oracle(m, x, y, passes)[..., :3], g[f"p{passes}_{name}"][..., :3]).all(), passes
 
 
-@need_ref
 def test_oracle_equals_reference_on_other_seeds_and_a_dark_frame():
     for seed in (1, 2):
         m, x, y = mu.case("roi2", seed)

@@ -18,11 +18,8 @@ def _build():
     util.build_oracle()
 
 
-need_ref = pytest.mark.skipif(util.ref("strict") is None and not os.path.isdir("/root/reference/src"),
-                              reason="oracle/_ref not built (no /root/reference)")
 
 
-@need_ref
 @pytest.mark.parametrize("name", list(util.BAYER))
 @pytest.mark.parametrize("size", [(16, 16), (117, 131), (206, 206), (207, 113), (1024, 768)])
 def test_rcd_oracle_equals_reference_strict(name, size):
@@ -38,7 +35,6 @@ def test_rcd_oracle_equals_reference_strict(name, size):
     assert (mask & 1).sum() < 4 * (w + h)
 
 
-@need_ref
 def test_rcd_reference_undefined_pixels_are_real():
     """The masked set is where the reference itself is not a function of its input: poisoning its
     uninitialised scratch moves (some of) those pixels and nothing else."""
@@ -52,21 +48,20 @@ def test_rcd_reference_undefined_pixels_are_real():
     assert not (moved & ((mask & 1) == 0)).any()
 
 
-@need_ref
+@pytest.mark.skipif(util.ref("fast") is None, reason="compares the reference's release build with its strict build: needs oracle/_ref")
 def test_rcd_fast_build_distance_is_what_design_md_says():
     """The release (-ffast-math) build of the SAME reference source is not within 1 ulp of its own
     strict build; record the distribution the parity statement in DESIGN.md quotes."""
     m = util.frame_natural(1024, 768, util.SEEDS[0])
     f = util.BAYER["RGGB"]
-    s = util.ref_rcd(m, f, kind="strict")
-    q = util.ref_rcd(m, f, kind="fast")
+    s = util.ref_rcd.__wrapped__(m, f, kind="strict")
+    q = util.ref_rcd.__wrapped__(m, f, kind="fast")
     mask = util.oracle_rcd_mask(m, f)
     u = util.ulp_distance(s[..., :3], q[..., :3])[(mask & 1) == 0]
     assert (u > 1).mean() > 0.01          # the release build is NOT within 1 ulp of the source semantics
     assert np.abs(s[..., :3] - q[..., :3])[(mask & 1) == 0].max() < 1e-3
 
 
-@need_ref
 @pytest.mark.parametrize("kind,fp", [("strict", util.FP_STRICT), ("fast", util.FP_CONTRACT)])
 def test_colour_oracle_equals_reference(kind, fp):
     enc, dec = util.srgb_encode_lut(), util.srgb_decode_lut()
@@ -82,7 +77,6 @@ def test_colour_oracle_equals_reference(kind, fp):
         assert same_bits(r, o).all()
 
 
-@need_ref
 @pytest.mark.parametrize("scale", [0, 2, 5])
 def test_eaw_oracle_equals_reference_strict(scale):
     rng = np.random.default_rng(scale)
@@ -130,13 +124,43 @@ def test_eaw_oracle_equals_golden():
     assert same_bits(util.oracle_eaw_synthesize(g["img"], g["detail_0"], tuple(g["thr"])), g["synth"]).all()
 
 
-@need_ref
+@util.recorded(lambda color_mode, new_vst, img, fwd, plan, oracle_back: (fwd, oracle_back))
+def _ref_dn_vst(color_mode, new_vst, img, fwd, plan, oracle_back):
+    """the reference's forward and inverse transforms of `img` / `fwd` with the parameters of the oracle's plan (the oracle's
+    results, `fwd` and `oracle_back`, are what a recording is stored against)"""
+    R, f4 = util.ref("strict"), (lambda v: (C.c_float * 4)(*v))
+    h, w = img.shape[:2]
+    wb, p, a_eff, b, bias = plan[1:5], plan[5:9], plan[9], plan[10], plan[11]
+    toY, toRGB, aa, bb = plan[12:24].copy(), plan[24:36].copy(), plan[36:40], plan[40:44]
+    rf, rb = np.zeros_like(img), fwd.copy()
+    if not new_vst:
+        R.ref_dn_precondition(util.fptr(img), util.fptr(rf), w, h, f4(aa), f4(bb))
+        R.ref_dn_backtransform(util.fptr(rb), w, h, f4(aa), f4(bb))
+    elif color_mode == 0:
+        R.ref_dn_precondition_v2(util.fptr(img), util.fptr(rf), w, h, C.c_float(a_eff), f4(p), C.c_float(b), f4(wb))
+        R.ref_dn_backtransform_v2(util.fptr(rb), w, h, C.c_float(a_eff), f4(p), C.c_float(b), C.c_float(bias), f4(wb))
+    else:
+        R.ref_dn_precondition_Y0U0V0(util.fptr(img), util.fptr(rf), w, h, C.c_float(a_eff), f4(p), C.c_float(b), util.fptr(toY))
+        R.ref_dn_backtransform_Y0U0V0(util.fptr(rb), w, h, C.c_float(a_eff), f4(p), C.c_float(b), C.c_float(bias), f4(wb), util.fptr(toRGB))
+    return rf, rb
+
+
+@util.recorded()
+def _ref_dn_call(fn, out_sizes, *args):
+    """one of the reference's denoise helpers: float32 outputs of `out_sizes` first, then `args` (4-tuples become float[4],
+    float32 arrays pointers)"""
+    outs = [np.zeros(n, np.float32) for n in out_sizes]
+    conv = [(C.c_float * 4)(*a) if isinstance(a, tuple) else util.fptr(a) if isinstance(a, np.ndarray) else a for a in args]
+    getattr(util.ref("strict"), fn)(*[util.fptr(o) for o in outs], *conv)
+    return tuple(outs)
+
+
 @pytest.mark.parametrize("color_mode,new_vst", [(1, True), (0, True), (0, False)])
 def test_denoise_vst_oracle_equals_reference(color_mode, new_vst):
     """precondition/backtransform{,_v2,_Y0U0V0} cut verbatim from iop/denoiseprofile.c:852-1089."""
     import ctypes as C
     import ansel_b200 as ab
-    O, R = util.oracle(), util.ref("strict")
+    O = util.oracle()
     f4 = lambda v: (C.c_float * 4)(*v)  # noqa: E731
     wbc, pm = (2.0, 1.0, 1.5, 0.0), (1.0, 1.0, 1.0, 1.0)
     img = util.rgba_scene(300, 200, 1)
@@ -145,41 +169,26 @@ def test_denoise_vst_oracle_equals_reference(color_mode, new_vst):
     d = ab.denoiseprofile_data(ab.DENOISE_WAVELETS, color_mode=color_mode, use_new_vst=new_vst, b=(0.0, 1e-6, 0.0))
     plan = np.zeros(51, np.float32)
     O.orc_dn_plan_export(C.byref(d), C.c_float(1.0), 6000, 4000, f4(wbc), f4(pm), util.fptr(plan))
-    wb, p, a_eff, b, bias = plan[1:5], plan[5:9], plan[9], plan[10], plan[11]
-    toY, toRGB, aa, bb = plan[12:24].copy(), plan[24:36].copy(), plan[36:40], plan[40:44]
     fwd, back = np.zeros_like(img), np.zeros_like(img)
     O.orc_dn_vst(1, C.byref(d), C.c_float(1.0), 6000, 4000, f4(wbc), f4(pm), util.fptr(img), util.fptr(fwd), C.c_size_t(npx))
     O.orc_dn_vst(0, C.byref(d), C.c_float(1.0), 6000, 4000, f4(wbc), f4(pm), util.fptr(fwd), util.fptr(back), C.c_size_t(npx))
-    rf, rb = np.zeros_like(img), fwd.copy()
-    if not new_vst:
-        R.ref_dn_precondition(util.fptr(img), util.fptr(rf), 300, 200, f4(aa), f4(bb))
-        R.ref_dn_backtransform(util.fptr(rb), 300, 200, f4(aa), f4(bb))
-    elif color_mode == 0:
-        R.ref_dn_precondition_v2(util.fptr(img), util.fptr(rf), 300, 200, C.c_float(a_eff), f4(p), C.c_float(b), f4(wb))
-        R.ref_dn_backtransform_v2(util.fptr(rb), 300, 200, C.c_float(a_eff), f4(p), C.c_float(b), C.c_float(bias), f4(wb))
-    else:
-        R.ref_dn_precondition_Y0U0V0(util.fptr(img), util.fptr(rf), 300, 200, C.c_float(a_eff), f4(p), C.c_float(b), util.fptr(toY))
-        R.ref_dn_backtransform_Y0U0V0(util.fptr(rb), 300, 200, C.c_float(a_eff), f4(p), C.c_float(b), C.c_float(bias), f4(wb),
-                                      util.fptr(toRGB))
+    rf, rb = _ref_dn_vst(color_mode, new_vst, img, fwd, plan, back)
     assert same_bits(fwd, rf).all() and same_bits(back, rb).all()
     assert np.abs(back[..., :3] - img[..., :3]).max() < 1e-3  # the pair is (nearly) an inverse
 
 
-@need_ref
 def test_denoise_plan_pieces_equal_reference():
     """compute_wb_factors, set_up_conversion_matrices, variance_stabilizing_xform (denoiseprofile.c:1098-1286)."""
     import ctypes as C
     import ansel_b200 as ab
-    O, R = util.oracle(), util.ref("strict")
+    O = util.oracle()
     f4 = lambda v: (C.c_float * 4)(*v)  # noqa: E731
     wbc, pm = (2.0, 1.0, 1.5, 0.0), (1.0, 1.0, 1.0, 1.0)
     d = ab.denoiseprofile_data(ab.DENOISE_WAVELETS)
-    a, b = np.zeros(4, np.float32), np.zeros(4, np.float32)
+    a = np.zeros(4, np.float32)
     O.orc_dn_wb_factors(util.fptr(a), C.byref(d), f4(wbc), f4(pm), f4((2, 1, 2, 0)))
-    R.ref_dn_wb_factors(util.fptr(b), 1, 1, f4(wbc), f4(pm), f4((2, 1, 2, 0)))
-    assert same_bits(a, b).all()
-    tY, tR = np.zeros(12, np.float32), np.zeros(12, np.float32)
-    R.ref_dn_conversion_matrices(util.fptr(tY), util.fptr(tR), f4(a))
+    assert same_bits(a, _ref_dn_call("ref_dn_wb_factors", (4,), 1, 1, wbc, pm, (2, 1, 2, 0))[0]).all()
+    tY, tR = _ref_dn_call("ref_dn_conversion_matrices", (12, 12), a)
     plan = np.zeros(51, np.float32)
     O.orc_dn_plan_export(C.byref(d), C.c_float(1.0), 6000, 4000, f4(wbc), f4(pm), util.fptr(plan))
     k = np.float32(d.strength) * np.float32(2.5) * np.float32(1.0)
@@ -188,11 +197,10 @@ def test_denoise_plan_pieces_equal_reference():
     force = np.ascontiguousarray(np.array(d.force, np.float32))
     for cm in (0, 1):
         d.wavelet_color_mode = cm
-        t1, t2 = np.zeros(4, np.float32), np.zeros(4, np.float32)
-        sums = f4((3e7, 2.5e7, 2.8e7, 1.0))
-        O.orc_wavelet_thresholds(util.fptr(t1), 2, 7, C.c_size_t(45441024), sums, C.c_float(plan[46]), C.byref(d))
-        R.ref_dn_thresholds(util.fptr(t2), 2, 7, C.c_size_t(45441024), sums, cm, util.fptr(force))
-        assert same_bits(t1, t2).all()
+        t1 = np.zeros(4, np.float32)
+        sums = (3e7, 2.5e7, 2.8e7, 1.0)
+        O.orc_wavelet_thresholds(util.fptr(t1), 2, 7, C.c_size_t(45441024), f4(sums), C.c_float(plan[46]), C.byref(d))
+        assert same_bits(t1, _ref_dn_call("ref_dn_thresholds", (4,), 2, 7, C.c_size_t(45441024), sums, cm, force)[0]).all()
 
 
 FILMIC_CASES = {"default_v8": {}, "no_bleach": dict(version=5), "high_bleach_hue": dict(version=8, saturation=60.0),
@@ -200,7 +208,6 @@ FILMIC_CASES = {"default_v8": {}, "no_bleach": dict(version=5), "high_bleach_hue
                 "wide_dr_gamma22": dict(white_point_source=6.0, black_point_source=-10.0, output_power=2.2)}
 
 
-@need_ref
 @pytest.mark.parametrize("name", list(FILMIC_CASES))
 def test_filmic_oracle_equals_reference(name):
     """filmic_agx and everything under it, cut verbatim from iop/filmicrgb.c:948-2649; piece->data from the
@@ -211,7 +218,7 @@ def test_filmic_oracle_equals_reference(name):
     for e in (export, None):
         assert same_bits(util.ref_filmic_agx(img, blob, work, e), util.oracle_filmic_agx(img, blob, work, e)).all()
     for v in (5, 6, 7, 8, 9):
-        assert same_bits(util.filmic_prepare(util.ref("strict"), "ref_filmic_prepare", v, work, export),
+        assert same_bits(util.ref_filmic_prepare(v, work, export),
                          util.filmic_prepare(util.oracle(), "orc_filmic_prepare", v, work, export)).all()
 
 
@@ -228,21 +235,15 @@ def test_filmic_abi_layout_matches_reference():
     import ctypes as C
     import ansel_b200 as ab
     assert C.sizeof(ab.FilmicPiece) == 1088
-    r = util.ref("strict")
-    if r is None:
-        pytest.skip("oracle/_ref not built")
     for fn, want in (("ref_filmic_sizeof_data", 832), ("ref_filmic_offsetof_spline", 128), ("ref_filmic_sizeof_spline", 144),
                      ("ref_filmic_offsetof_noise_distribution", 272), ("ref_filmic_sizeof_params", 112)):
-        f = getattr(r, fn)
-        f.restype = C.c_size_t
-        assert f() == want
+        assert util.ref_size_t(fn) == want
 
 
 NLM_CONFIGS = [dict(), dict(P=2, K=4, scattering=0.5), dict(center_weight=-1.0, sharpness=0.01, luma=0.8, chroma=0.6, K=3, P=3),
                dict(K=2, P=1, scattering=1.0, scale=0.7), dict(P=4, K=2), dict(P=0, K=3), dict(K=5, decimate=1)]
 
 
-@need_ref
 @pytest.mark.parametrize("cfg", range(len(NLM_CONFIGS)))
 def test_nlmeans_oracle_equals_reference(cfg):
     """pixel/nlmeans_core.c compiled in place; chunked, order-dependent float accumulation."""
@@ -260,7 +261,6 @@ def test_nlmeans_oracle_equals_golden():
 LL_PARAMS = [dict(), dict(sigma=0.2, shadows=1.5, highlights=0.1, clarity=1.0), dict(sigma=0.8, shadows=-0.5, highlights=1.8, clarity=-0.6)]
 
 
-@need_ref
 @pytest.mark.parametrize("p", range(len(LL_PARAMS)))
 def test_local_laplacian_oracle_equals_reference(p):
     """pixel/locallaplacian.c compiled in place; channel 0 is the filter output, 1,2 copies, 3 untouched."""
@@ -290,7 +290,6 @@ def _diffuse_cases():
     return out
 
 
-@need_ref
 @pytest.mark.parametrize("name", list(_diffuse_cases()))
 def test_diffuse_oracle_equals_reference(name):
     """iop/diffuse.c process() cut verbatim + pixel/bspline.h; NaN/inf/negative input included (hdr_rgba)."""
@@ -328,7 +327,6 @@ def test_libm_sinf_cosf_restatement_equals_system_libm():
 WORK_PROFILE = util.profile_pair(util.REC2020_TO_XYZ_D50)
 
 
-@need_ref
 def test_lab_glue_oracle_equals_reference():
     """colorprofiles/iop_profile.c _transform_rgb_to_lab_matrix / _transform_lab_to_rgb_matrix cut verbatim."""
     rgb = util.hdr_rgba(333, 217, 6)                     # negatives, zeros, NaN, inf, > 1
@@ -361,7 +359,6 @@ def _srgb_curves(partial):
     return d, util.fit_unbounded_coeffs(d), e, util.fit_unbounded_coeffs(e)
 
 
-@need_ref
 @pytest.mark.parametrize("partial", [False, True])
 def test_lab_glue_with_tone_curves_oracle_equals_reference(partial):
     """_apply_tonecurves + the two matrix loops cut verbatim, for a profile with tone curves (sRGB)"""
@@ -376,7 +373,6 @@ def test_lab_glue_with_tone_curves_oracle_equals_reference(partial):
     assert same_bits(util.ref_rgb_to_lab_trc(rgb, SRGB_PROFILE, d, cd, e, ce), util.ref_rgb_to_lab(rgb, SRGB_PROFILE)).all()
 
 
-@need_ref
 @pytest.mark.parametrize("scale,pipe,prev", [(1.0, 1, 0), (0.5, 1, 0), (2.5, 2, 0), (0.3, 4, 0), (0.4, 3, 1)])
 def test_nlmeans_iop_oracle_equals_reference(scale, pipe, prev):
     """iop/nlmeans.c process_cpu cut verbatim: P, K, sharpness, Lab norms, decimation, mask alpha copy."""
@@ -390,7 +386,6 @@ def test_nlmeans_iop_oracle_equals_reference(scale, pipe, prev):
             assert same_bits(got, want).all()
 
 
-@need_ref
 @pytest.mark.parametrize("passes", [1, 3, 5])
 def test_color_smoothing_oracle_equals_reference(passes):
     """iop/demosaic/basic.c color_smoothing cut verbatim (median network, alpha lane as scratch)."""
@@ -399,7 +394,6 @@ def test_color_smoothing_oracle_equals_reference(passes):
         assert same_bits(util.oracle_color_smoothing(img, passes), util.ref_color_smoothing(img, passes)).all()
 
 
-@need_ref
 @pytest.mark.parametrize("name", list(util.BAYER))
 @pytest.mark.parametrize("mode", [1, 2, 3])
 def test_green_eq_oracle_equals_reference(name, mode):
@@ -425,7 +419,6 @@ def test_demosaic_extras_oracle_equals_golden():
 LEGACY_EXTRA = [{}, dict(saturation=20.0), dict(saturation=-15.0, shadows=0, highlights=2, contrast=1.4)]
 
 
-@need_ref
 @pytest.mark.parametrize("version", [0, 1, 2, 3, 4])
 def test_filmic_legacy_oracle_equals_reference(version):
     """filmic_split/chroma_v1, _v2_v3, _v4 and filmic_v5 cut verbatim from filmicrgb.c, every norm, with/without an
@@ -447,7 +440,6 @@ def test_filmic_legacy_oracle_equals_golden():
         assert same_bits(util.oracle_filmic_legacy(g["img"], g["data_" + tag], work, export), g[key]).all(), tag
 
 
-@need_ref
 @pytest.mark.parametrize("name", list(util.BAYER))
 def test_amaze_oracle_equals_reference(name):
     """iop/demosaic/amaze.cc compiled in place, one thread (its scratch is carried from tile to tile in raster order:
@@ -458,7 +450,6 @@ def test_amaze_oracle_equals_reference(name):
         assert same_bits(util.oracle_amaze(m, f, pm, 0), util.ref_amaze(m, f, pm)).all()
 
 
-@need_ref
 def test_amaze_edge_inputs_and_scratch_modes():
     f = util.BAYER["RGGB"]
     for kind in ("zeros", "ones", "impulses", "negative", "tiny"):
@@ -493,7 +484,6 @@ def _reconstruct_frames():
             "dark": (util.rgba_scene(100, 80, 4) * 0.01).astype(np.float32), "tiny": (util.rgba_scene(7, 5, 4) * 3).astype(np.float32)}
 
 
-@need_ref
 @pytest.mark.parametrize("name", list(RECONSTRUCT_CASES))
 def test_filmic_reconstruct_oracle_equals_reference(name):
     """process() :2729-2838 replayed on mask_clipped_pixels / inpaint_noise / reconstruct_highlights / compute_ratios /
@@ -514,14 +504,28 @@ def test_filmic_reconstruct_oracle_equals_golden():
         assert rc == 1 and same_bits(frame, g["frame_" + name]).all() and same_bits(mask, g["mask_" + name]).all()
 
 
-@need_ref
+@util.recorded(lambda img, plan, center_weight, oracle_out: oracle_out)
+def _ref_dn_nlmeans_module(img, plan, center_weight, oracle_out):
+    """precondition_v2 -> nlmeans_denoise -> backtransform_v2 of the reference, with the parameters of the oracle's plan (the
+    oracle's module output `oracle_out` is what a recording is stored against)"""
+    R, f4 = util.ref("strict"), (lambda v: (C.c_float * 4)(*v))
+    h, w = img.shape[:2]
+    wb, p, a_eff, b, bias = plan[1:5], plan[5:9], plan[9], plan[10], plan[11]
+    pre = np.zeros_like(img)
+    R.ref_dn_precondition_v2(util.fptr(img), util.fptr(pre), w, h, C.c_float(a_eff), f4(p), C.c_float(b), f4(wb))
+    nlm = util.ref_nlmeans(pre, kind="strict", sharpness=float(np.float32(0.045) / np.float32(9)), center_weight=center_weight, P=1, K=7)
+    buf = np.ascontiguousarray(nlm)
+    R.ref_dn_backtransform_v2(util.fptr(buf), w, h, C.c_float(a_eff), f4(p), C.c_float(b), C.c_float(bias), f4(wb))
+    return buf
+
+
 def test_denoiseprofile_nlmeans_module_is_the_reference_pieces_in_order():
     """process_nlmeans_cpu(), denoiseprofile.c:1599-1648, composed from the reference's own precondition_v2, nlmeans_denoise and
     backtransform_v2 with the parameters nlmeans_precondition() :1500-1533 derives (exported by the oracle's NLM plan): what
     bench.py's CPU arm runs for the denoise node of the C3 chain, and what the oracle's module-level entry point restates"""
     import ctypes as C
     import ansel_b200 as ab
-    O, R = util.oracle(), util.ref("strict")
+    O = util.oracle()
     f4 = lambda v: (C.c_float * 4)(*v)  # noqa: E731
     w, h = 300, 200
     img = util.rgba_scene(w, h, 5)
@@ -529,14 +533,9 @@ def test_denoiseprofile_nlmeans_module_is_the_reference_pieces_in_order():
     wbc, pm = (2.0, 1.0, 1.5, 0.0), (1.0, 1.0, 1.0, 1.0)
     plan = np.zeros(51, np.float32)
     O.orc_dn_plan_export_nlm(C.byref(d), C.c_float(1.0), w, h, f4(wbc), f4(pm), util.fptr(plan))
-    wb, p, a_eff, b, bias = plan[1:5], plan[5:9], plan[9], plan[10], plan[11]
-    pre = np.zeros_like(img)
-    R.ref_dn_precondition_v2(util.fptr(img), util.fptr(pre), w, h, C.c_float(a_eff), f4(p), C.c_float(b), f4(wb))
-    nlm = util.ref_nlmeans(pre, kind="strict", sharpness=float(np.float32(0.045) / np.float32(9)), center_weight=float(np.float32(d.central_pixel_weight)), P=1, K=7)
-    buf = np.ascontiguousarray(nlm)
-    R.ref_dn_backtransform_v2(util.fptr(buf), w, h, C.c_float(a_eff), f4(p), C.c_float(b), C.c_float(bias), f4(wb))
     f = O.orc_denoiseprofile_nlmeans
     f.restype = C.c_int
     want = np.zeros_like(img)
     assert f(util.fptr(img), util.fptr(want), w, h, C.byref(d), C.c_float(1.0), 1, f4(wbc), f4(pm)) == 0
+    buf = _ref_dn_nlmeans_module(img, plan, float(np.float32(d.central_pixel_weight)), want)
     assert same_bits(buf, want).all()

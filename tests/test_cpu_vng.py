@@ -23,11 +23,9 @@ def _build():
         util.build_oracle()
 
 
-need_ref = pytest.mark.skipif(util.ref("strict") is None and not os.path.isdir("/root/reference/src"), reason="oracle/_ref not built (no /root/reference)")
 THRESHOLDS = (0.2, 0.05, 1.0)
 
 
-@need_ref
 @pytest.mark.parametrize("name", list(vu.CASES))
 def test_vng_oracle_equals_reference(name):
     m, filters, x, y = vu.case(name)
@@ -35,7 +33,6 @@ def test_vng_oracle_equals_reference(name):
         assert same_bits(vu.oracle_vng(m, filters, x, y, lin), vu.ref_vng(m, filters, x, y, lin)).all(), lin
 
 
-@need_ref
 @pytest.mark.parametrize("name", list(vu.CASES))
 def test_dual_oracle_equals_reference(name):
     m, filters, x, y = vu.case(name)
@@ -71,7 +68,6 @@ def test_dual_kernels_equal_oracle(name):
         assert same_bits(vu.emul_dual(rgb, m, filters, x, y, thr), vu.oracle_dual(rgb, m, filters, x, y, thr)).all(), thr
 
 
-@need_ref
 @pytest.mark.parametrize("name", list(vu.XTRANS_CASES))
 def test_vng_xtrans_oracle_equals_reference(name):
     """the X-Trans branch of vng_interpolate (three colours, 6x6 periods); lane 3 is uninitialised memory in the reference"""

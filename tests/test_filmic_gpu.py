@@ -22,11 +22,10 @@ def same_bits(a, b):
 
 
 def data_blob(name):
-    """dt_iop_filmicrgb_data_t for a case: the reference's commit_params() here, the golden copy on the GPU box."""
+    """dt_iop_filmicrgb_data_t for a case: the golden copy, checked against the reference's commit_params()."""
     g = np.load(os.path.join(util.GOLDEN_DIR, "filmic_data.npz"))
-    if util.ref("strict") is not None:
-        live = util.ref_filmic_commit(util.filmic_default_params(**CASES[name]))
-        assert (live == g[name]).all(), "committed filmic_data.npz is stale"
+    live = util.ref_filmic_commit(util.filmic_default_params(**CASES[name]))
+    assert (live == g[name]).all(), "committed filmic_data.npz is stale"
     return g[name]
 
 
@@ -114,11 +113,13 @@ def test_filmic_legacy_golden_and_host(built):
         assert same_bits(got[..., :lanes], g["out_" + tag][..., :lanes]).all(), tag
 
 
-@pytest.mark.skipif(util.ref("strict") is None, reason="needs the reference build (authoring container)")
+def legacy_live_blobs():
+    return {(version, pc): util.ref_filmic_commit(util.filmic_default_params(version=version, preserve_color=pc, saturation=-15.0, shadows=0, highlights=2))
+            for version in range(5) for pc in range(6)}
+
+
 def test_filmic_legacy_all_norms_live(built):
-    """where the reference is present: every version x norm x parameter set from its own commit_params()"""
+    """every version x norm x parameter set from the reference's own commit_params()"""
     img = util.hdr_rgba(320, 200, 3)
-    for version in range(5):
-        for pc in range(6):
-            blob = util.ref_filmic_commit(util.filmic_default_params(version=version, preserve_color=pc, saturation=-15.0, shadows=0, highlights=2))
-            assert same_bits(cuda_filmic(img, blob, EXPORT), util.oracle_filmic_legacy(img, blob, WORK, EXPORT)).all(), (version, pc)
+    for (version, pc), blob in legacy_live_blobs().items():
+        assert same_bits(cuda_filmic(img, blob, EXPORT), util.oracle_filmic_legacy(img, blob, WORK, EXPORT)).all(), (version, pc)

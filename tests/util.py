@@ -44,12 +44,206 @@ def oracle() -> C.CDLL:
 
 
 def ref(kind: str = "strict"):
-    """oracle/_ref/libref_{strict,fast}.so or None when it was never built (no /root/reference)."""
+    """oracle/_ref/libref_{strict,fast}.so or None when it was never built (the reference sources are absent)."""
     key = "ref_" + kind
     if key not in _cache:
         path = os.path.join(ORACLE_DIR, "_ref", f"libref_{kind}.so")
         _cache[key] = C.CDLL(path) if os.path.exists(path) else None
     return _cache[key]
+
+
+# ---- the reference's outputs, recorded ----------------------------------------------------------------------------------
+# oracle/_ref can only be built where the reference sources are.  Every helper that calls into it is wrapped by
+# `recorded`: with the library present it runs the reference; without it, it returns what the reference returned for the
+# same arguments, read from tests/golden/reference/ (written by tests/golden/make_golden_reference.py).  The arguments are
+# fingerprinted by content, so a test whose inputs change no longer finds a recording and fails instead of comparing
+# against a stale output.  `candidate` (optional) computes the same outputs with the oracle: the recording then keeps only
+# the elements where the reference differs from it plus a SHA-256 of the reference's bytes, and the replay checks that
+# digest, so what it returns is bit for bit what the reference returned.
+RECORD_DIR = os.path.join(GOLDEN_DIR, "reference")
+RECORDING = os.environ.get("B200_RECORD_REFERENCE") == "1"
+_records, _recorded_now = {}, {}
+
+
+def _fingerprint(h, v) -> None:
+    if isinstance(v, np.ndarray):
+        h.update(f"a{v.dtype.str}{v.shape}".encode())
+        h.update(np.ascontiguousarray(v).tobytes())
+    elif isinstance(v, (C.Structure, C.Union)):
+        h.update(type(v).__name__.encode())
+        if isinstance(getattr(v, "_keepalive", None), (C.Structure, C.Union, C.Array)):   # the data a piece points at (ansel_b200.make_piece)
+            _fingerprint(h, v._keepalive)
+        for field in v._fields_:
+            name, typ = field[0], field[1]
+            while issubclass(typ, C.Array):
+                typ = typ._type_
+            if issubclass(typ, (C._Pointer, C.c_void_p, C.c_char_p, C._CFuncPtr)):
+                h.update(b"*")          # an address is not content; what a piece points at is fingerprinted by the caller's arrays
+            else:
+                _fingerprint(h, getattr(v, name))
+    elif isinstance(v, C.Array):
+        h.update(b"[")
+        for x in v:
+            _fingerprint(h, x)
+    elif isinstance(v, (list, tuple)):
+        h.update(b"(%d" % len(v))
+        for x in v:
+            _fingerprint(h, x)
+    elif isinstance(v, dict):
+        h.update(b"{")
+        for k in sorted(v):
+            h.update(repr(k).encode())
+            _fingerprint(h, v[k])
+    elif isinstance(v, C._SimpleCData):
+        h.update(type(v).__name__.encode() + repr(v.value).encode())
+    elif isinstance(v, np.generic):
+        h.update(v.dtype.str.encode() + v.tobytes())
+    elif v is None or isinstance(v, (bool, int, float, str, bytes)):
+        h.update(repr(v).encode())
+    else:
+        raise TypeError(f"recorded: cannot fingerprint an argument of type {type(v).__name__}")
+
+
+def _flatten(obj, leaves):
+    if isinstance(obj, tuple):
+        return ["t"] + [_flatten(x, leaves) for x in obj]
+    if obj is None:
+        return None
+    leaves.append(np.asarray(obj))
+    return len(leaves) - 1
+
+
+def _unflatten(spec, leaves):
+    if isinstance(spec, list):
+        return tuple(_unflatten(x, leaves) for x in spec[1:])
+    if spec is None:
+        return None
+    a = leaves[spec]
+    return a if a.ndim else a[()]
+
+
+def _raw(a: np.ndarray) -> np.ndarray:
+    return np.ascontiguousarray(a).reshape(-1).view(f"u{a.dtype.itemsize}") if a.dtype.itemsize in (1, 2, 4, 8) else None
+
+
+def _store(name: str, key: str, out, cand) -> None:
+    import hashlib
+    import json
+    leaves, cleaves = [], []
+    spec = _flatten(out, leaves)
+    if cand is not None:
+        _flatten(cand, cleaves)
+    entry = {key: np.array(json.dumps([spec, len(leaves)]))}
+    for i, a in enumerate(leaves):
+        c = cleaves[i] if i < len(cleaves) else None
+        if a.ndim and c is not None and c.shape == a.shape and c.dtype == a.dtype and _raw(a) is not None:
+            ra, rc = _raw(a), _raw(c)
+            idx = np.flatnonzero(ra != rc)
+            entry[f"{key}.{i}.sha"] = np.array(hashlib.sha256(ra.tobytes()).hexdigest())
+            entry[f"{key}.{i}.shape"] = np.array(a.shape, np.int64)
+            entry[f"{key}.{i}.idx"] = idx.astype(np.int32 if ra.size < 2 ** 31 else np.int64)
+            entry[f"{key}.{i}.val"] = ra[idx]
+        else:
+            entry[f"{key}.{i}"] = a
+    _recorded_now.setdefault(name, {}).update(entry)
+
+
+def _load(name: str, key: str, cand_fn, args, kwargs):
+    import hashlib
+    import json
+    if name not in _records:
+        _records[name] = {}
+        for path in _record_files(name):
+            _records[name].update(np.load(path))
+    rec = _records[name]
+    if key not in rec:
+        raise AssertionError(f"{name}: the reference is not built here and these arguments were never recorded "
+                             "(tests/golden/make_golden_reference.py records them where the reference sources are)")
+    spec, n = json.loads(str(rec[key]))
+    cleaves = None
+    leaves = []
+    for i in range(n):
+        if f"{key}.{i}" in rec:
+            leaves.append(rec[f"{key}.{i}"])
+            continue
+        if cleaves is None:
+            cleaves = []
+            _flatten(cand_fn(*args, **kwargs), cleaves)
+        c = np.array(cleaves[i])
+        assert tuple(c.shape) == tuple(rec[f"{key}.{i}.shape"]), f"{name}: the oracle's output no longer has the recorded shape"
+        rc = _raw(c)
+        rc[rec[f"{key}.{i}.idx"]] = rec[f"{key}.{i}.val"]
+        assert hashlib.sha256(rc.tobytes()).hexdigest() == str(rec[f"{key}.{i}.sha"]), (
+            f"{name}: the oracle plus the recorded differences no longer rebuilds the reference's output "
+            "(the oracle changed where it used to equal the reference)")
+        leaves.append(c)
+    return _unflatten(spec, leaves)
+
+
+def recorded(candidate=None):
+    """wrap a helper that calls oracle/_ref (see the comment above); `candidate` takes the helper's arguments"""
+    import functools
+    import hashlib
+    import inspect
+
+    def wrap(fn):
+        sig = inspect.signature(fn)
+        name = f"{fn.__module__}.{fn.__name__}"
+
+        @functools.wraps(fn)
+        def call(*args, **kwargs):
+            bound = sig.bind(*args, **kwargs)
+            bound.apply_defaults()
+            h = hashlib.sha256(name.encode())
+            _fingerprint(h, dict(bound.arguments))
+            key = h.hexdigest()[:24]
+            if ref(bound.arguments.get("kind", "strict")) is None:
+                return _load(name, key, candidate, args, kwargs)
+            out = fn(*args, **kwargs)
+            if RECORDING:
+                _store(name, key, out, candidate(*args, **kwargs) if candidate else None)
+            return out
+        return call
+    return wrap
+
+
+def _save_recordings() -> None:
+    """merge what this process recorded into tests/golden/reference/<helper>[.<shard>].npz, each file under 1 MB"""
+    import io
+    os.makedirs(RECORD_DIR, exist_ok=True)
+    for name, entry in _recorded_now.items():
+        old = {}
+        for path in _record_files(name):
+            old.update(np.load(path))
+            os.remove(path)
+        old.update(entry)
+        n = 1
+        while True:
+            shards = [{k: v for k, v in old.items() if int(k[:6], 16) % n == i} for i in range(n)]
+            blobs = []
+            for shard in shards:
+                buf = io.BytesIO()
+                np.savez_compressed(buf, **shard)
+                blobs.append(buf.getvalue())
+            if max(len(b) for b in blobs) < 900_000:
+                break
+            n *= 2
+        for i, blob in enumerate(blobs):
+            with open(os.path.join(RECORD_DIR, f"{name}.npz" if n == 1 else f"{name}.{i}.npz"), "wb") as f:
+                f.write(blob)
+
+
+def _record_files(name: str):
+    import glob
+    return sorted(glob.glob(os.path.join(RECORD_DIR, glob.escape(name) + ".npz")) + glob.glob(os.path.join(RECORD_DIR, glob.escape(name) + ".[0-9]*.npz")))
+
+
+@recorded()
+def ref_size_t(fn: str, *args: int, kind: str = "strict") -> int:
+    """a size or offset the reference's compiler gives (the ref_sizeof_* / ref_offsetof_* exports of oracle/_ref)"""
+    f = getattr(ref(kind), fn)
+    f.restype = C.c_size_t
+    return int(f(*args))
 
 
 def fptr(a: np.ndarray):
@@ -88,6 +282,7 @@ def oracle_rcd_mask(mosaic: np.ndarray, filters: int, pm=(1.0, 1.0, 1.0)) -> np.
     return mask
 
 
+@recorded(lambda mosaic, filters, pm=(1.0, 1.0, 1.0), kind="strict", poison=0.0: oracle_rcd(mosaic, filters, pm))
 def ref_rcd(mosaic: np.ndarray, filters: int, pm=(1.0, 1.0, 1.0), kind: str = "strict", poison: float = 0.0):
     lib = ref(kind)
     if lib is None:
@@ -263,6 +458,8 @@ def oracle_convert(rgba, matrix, clip=None, lut_s=None, co_s=None, lut_t=None, c
     return np.array(dst)
 
 
+@recorded(lambda rgba, matrix, clip=None, lut_s=None, co_s=None, lut_t=None, co_t=None, kind="fast":
+          oracle_convert(rgba, matrix, clip, lut_s, co_s, lut_t, co_t, fp=FP_CONTRACT if kind == "fast" else FP_STRICT))
 def ref_convert(rgba, matrix, clip=None, lut_s=None, co_s=None, lut_t=None, co_t=None, kind="fast"):
     lib = ref(kind)
     if lib is None:
@@ -293,6 +490,7 @@ def oracle_eaw_decompose(img: np.ndarray, scale: int, inv_sigma2: float):
     return coarse, detail, np.array(list(sums))
 
 
+@recorded(lambda img, scale, inv_sigma2, kind="strict": oracle_eaw_decompose(img, scale, inv_sigma2))
 def ref_eaw_decompose(img: np.ndarray, scale: int, inv_sigma2: float, kind: str = "strict"):
     lib = ref(kind)
     if lib is None:
@@ -311,6 +509,7 @@ def oracle_eaw_synthesize(base: np.ndarray, detail: np.ndarray, thr, boost=(1, 1
     return out
 
 
+@recorded(lambda base, detail, thr, boost=(1, 1, 1, 1), kind="strict": oracle_eaw_synthesize(base, detail, thr, boost))
 def ref_eaw_synthesize(base, detail, thr, boost=(1, 1, 1, 1), kind="strict"):
     lib = ref(kind)
     if lib is None:
@@ -387,6 +586,7 @@ def filmic_params_blob(p: dict) -> np.ndarray:
     return blob
 
 
+@recorded()
 def ref_filmic_commit(params: dict, kind: str = "strict"):
     """dt_iop_filmicrgb_data_t (832 bytes) from the reference's own commit_params()."""
     lib = ref(kind)
@@ -405,6 +605,7 @@ def _f9(a):
     return fptr(np.ascontiguousarray(a, np.float32).reshape(-1).copy()) if a is not None else None
 
 
+@recorded(lambda rgba, data_blob, work, export=None, kind="strict": oracle_filmic_agx(rgba, data_blob, work, export))
 def ref_filmic_agx(rgba, data_blob, work, export=None, kind="strict"):
     lib = ref(kind)
     h, w = rgba.shape[:2]
@@ -430,6 +631,7 @@ def oracle_filmic_agx(rgba, data_blob, work, export=None):
     return dst
 
 
+@recorded(lambda rgba, data_blob, work, export=None, kind="strict": oracle_filmic_legacy(rgba, data_blob, work, export))
 def ref_filmic_legacy(rgba, data_blob, work, export=None, kind="strict"):
     """the v1..v5 colour sciences through the reference's own functions; lanes a branch does not write keep the input's"""
     lib = ref(kind)
@@ -471,6 +673,7 @@ def _filmic_reconstruct(lib, fn, rgba, data_blob, iscale, roi_scale, buf):
     return rc, np.array(dst), np.array(mask)
 
 
+@recorded(lambda rgba, data_blob, iscale=1.0, roi_scale=1.0, buf=None, kind="strict": oracle_filmic_reconstruct(rgba, data_blob, iscale, roi_scale, buf))
 def ref_filmic_reconstruct(rgba, data_blob, iscale=1.0, roi_scale=1.0, buf=None, kind="strict"):
     """process() :2729-2838 on the cut functions: (recovered?, frame the tone mapping reads, clipping mask)"""
     lib = ref(kind)
@@ -486,6 +689,11 @@ def filmic_prepare(lib, fn, version, work, export=None):
     keep = [_f9(work[0]), _f9(work[1]), _f9(export[0]) if export else None, _f9(export[1]) if export else None]
     getattr(lib, fn)(version, *keep, fptr(out))
     return out
+
+
+@recorded(lambda version, work, export=None, kind="strict": filmic_prepare(oracle(), "orc_filmic_prepare", version, work, export))
+def ref_filmic_prepare(version, work, export=None, kind="strict"):
+    return filmic_prepare(ref(kind), "ref_filmic_prepare", version, work, export)
 
 
 def hdr_rgba(w: int, h: int, seed: int) -> np.ndarray:
@@ -522,6 +730,7 @@ def oracle_nlmeans(img, *, scattering=0.0, scale=1.0, luma=1.0, chroma=1.0, cent
     return _nlm_call(oracle(), "orc_nlmeans_denoise", img, scattering, scale, luma, chroma, center_weight, sharpness, P, K, decimate, norm)
 
 
+@recorded(lambda img, kind="strict", **kw: oracle_nlmeans(img, **kw))
 def ref_nlmeans(img, kind="strict", **kw):
     lib = ref(kind)
     if lib is None:
@@ -563,6 +772,7 @@ def oracle_local_laplacian(img, sigma=0.5, shadows=0.5, highlights=0.5, clarity=
     return _ll_call(oracle(), "orc_local_laplacian", img, sigma, shadows, highlights, clarity)
 
 
+@recorded(lambda img, sigma=0.5, shadows=0.5, highlights=0.5, clarity=0.25, kind="strict": oracle_local_laplacian(img, sigma, shadows, highlights, clarity))
 def ref_local_laplacian(img, sigma=0.5, shadows=0.5, highlights=0.5, clarity=0.25, kind="strict"):
     lib = ref(kind)
     return None if lib is None else _ll_call(lib, "ref_local_laplacian", img, sigma, shadows, highlights, clarity)
@@ -586,6 +796,7 @@ def oracle_diffuse(img, data, iscale=1.0, roi_scale=1.0):
     return _diffuse_call(oracle(), "orc_diffuse", img, data, iscale, roi_scale)
 
 
+@recorded(lambda img, data, iscale=1.0, roi_scale=1.0, kind="strict": oracle_diffuse(img, data, iscale, roi_scale))
 def ref_diffuse(img, data, iscale=1.0, roi_scale=1.0, kind="strict"):
     lib = ref(kind)
     if lib is None:
@@ -617,11 +828,13 @@ def oracle_lab_to_rgb(img, work):
     return _glue(oracle(), "orc_lab_to_rgb", img, (work[1],), 1)
 
 
+@recorded(lambda img, work, kind="strict": oracle_rgb_to_lab(img, work))
 def ref_rgb_to_lab(img, work, kind="strict"):
     lib = ref(kind)
     return None if lib is None else _glue(lib, "ref_rgb_to_lab", img, work, 2)
 
 
+@recorded(lambda img, work, kind="strict": oracle_lab_to_rgb(img, work))
 def ref_lab_to_rgb(img, work, kind="strict"):
     lib = ref(kind)
     return None if lib is None else _glue(lib, "ref_lab_to_rgb", img, work, 2)
@@ -651,11 +864,14 @@ def oracle_lab_to_rgb_trc(img, work, lut_out, co_out):
     return _glue_trc(oracle(), "orc_lab_to_rgb_trc", img, (work[1],), (lut_out,), (co_out,))
 
 
+@recorded(lambda img, work, lut_in, co_in, lut_out, co_out, kind="strict": oracle_rgb_to_lab_trc(img, work, lut_in, co_in))
 def ref_rgb_to_lab_trc(img, work, lut_in, co_in, lut_out, co_out, kind="strict"):
     lib = ref(kind)
     return None if lib is None else _glue_trc(lib, "ref_rgb_to_lab_trc", img, work, (lut_in, lut_out), (co_in, co_out))
 
 
+@recorded(lambda img, work, lut_in, co_in, lut_out, co_out, kind="strict":
+          oracle_lab_to_rgb(img, work) if (lut_in[:, 0] < 0).all() else oracle_lab_to_rgb_trc(img, work, lut_out, co_out))
 def ref_lab_to_rgb_trc(img, work, lut_in, co_in, lut_out, co_out, kind="strict"):
     lib = ref(kind)
     return None if lib is None else _glue_trc(lib, "ref_lab_to_rgb_trc", img, work, (lut_in, lut_out), (co_in, co_out))
@@ -673,6 +889,8 @@ def oracle_nlmeans_iop(img, data, roi_scale=1.0, decimate=0, mask_display=0):
     return np.array(out)
 
 
+@recorded(lambda img, data, roi_scale=1.0, pipe_type=1, has_preview=0, mask_display=0, kind="strict":
+          oracle_nlmeans_iop(img, data, roi_scale, 1 if (pipe_type == 4 or has_preview) else 0, mask_display))
 def ref_nlmeans_iop(img, data, roi_scale=1.0, pipe_type=1, has_preview=0, mask_display=0, kind="strict"):
     lib = ref(kind)
     if lib is None:
@@ -715,6 +933,7 @@ def oracle_green_eq(mosaic, filters, mode, x=0, y=0, iso=100.0):
     return m
 
 
+@recorded(lambda mosaic, filters, mode, x=0, y=0, iso=100.0, kind="strict": oracle_green_eq(mosaic, filters, mode, x, y, iso))
 def ref_green_eq(mosaic, filters, mode, x=0, y=0, iso=100.0, kind="strict"):
     lib = ref(kind)
     if lib is None:
@@ -742,6 +961,7 @@ def oracle_color_smoothing(rgba, passes):
     return _smooth(oracle(), "orc_color_smoothing", rgba, passes)
 
 
+@recorded(lambda rgba, passes, kind="strict": oracle_color_smoothing(rgba, passes))
 def ref_color_smoothing(rgba, passes, kind="strict"):
     lib = ref(kind)
     return None if lib is None else _smooth(lib, "ref_color_smoothing", rgba, passes)
@@ -760,6 +980,7 @@ def oracle_amaze(mosaic, filters, pm=(1.0, 1.0, 1.0), scratch_mode=1):
     return out
 
 
+@recorded(lambda mosaic, filters, pm=(1.0, 1.0, 1.0), kind="strict", threads=1: oracle_amaze(mosaic, filters, pm, 0))
 def ref_amaze(mosaic, filters, pm=(1.0, 1.0, 1.0), kind="strict", threads=1):
     lib = ref(kind)
     if lib is None:
@@ -775,3 +996,8 @@ def ref_amaze(mosaic, filters, pm=(1.0, 1.0, 1.0), kind="strict", threads=1):
     lib.ref_amaze_demosaic(fptr(out), fptr(src), w, h, C.c_uint32(filters), (C.c_float * 3)(*pm))
     C.CDLL("libgomp.so.1").omp_set_num_threads(os.cpu_count() or 1)
     return np.array(out)
+
+
+if RECORDING:
+    import atexit
+    atexit.register(_save_recordings)

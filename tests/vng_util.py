@@ -47,6 +47,7 @@ def oracle_vng(m, filters, x=0, y=0, lin=0):
     return _vng(util.oracle(), "orc_vng_interpolate", m, filters, x, y, lin)
 
 
+@util.recorded(lambda m, filters, x=0, y=0, lin=0, kind="strict": oracle_vng(m, filters, x, y, lin))
 def ref_vng(m, filters, x=0, y=0, lin=0, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _vng(lib, "ref_vng_interpolate", m, filters, x, y, lin)
@@ -68,6 +69,7 @@ def oracle_dual(rgb, m, filters, x, y, thr, mask=0):
     return _dual(util.oracle(), "orc_dual_demosaic", rgb, m, filters, x, y, thr, mask)
 
 
+@util.recorded(lambda rgb, m, filters, x, y, thr, mask=0, kind="strict": oracle_dual(rgb, m, filters, x, y, thr, mask))
 def ref_dual(rgb, m, filters, x, y, thr, mask=0, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _dual(lib, "ref_dual_demosaic", rgb, m, filters, x, y, thr, mask)
@@ -140,6 +142,7 @@ def oracle_vng_xtrans(m, x=0, y=0, lin=0):
     return _vng_xtrans(util.oracle(), "orc_vng_interpolate_xtrans", m, x, y, lin)
 
 
+@util.recorded(lambda m, x=0, y=0, lin=0, kind="strict": oracle_vng_xtrans(m, x, y, lin))
 def ref_vng_xtrans(m, x=0, y=0, lin=0, kind="strict"):
     lib = util.ref(kind)
     return None if lib is None else _vng_xtrans(lib, "ref_vng_interpolate_xtrans", m, x, y, lin)
