@@ -20,6 +20,7 @@
 // in global memory; the row-sequential refinements stage their half plane in shared memory, the chain sweeps fetch the
 // operands of four steps at a time.
 #include "runtime.h"
+#include <atomic>
 #include <math.h>
 
 namespace
@@ -870,17 +871,19 @@ int amaze_demosaic_dev(const float *d_in, float *d_out, int width, int height, u
     a.ex = 1;
   }
   // persistent CTAs: as many as are resident at once (register-limited), each with its own scratch region
-  static int per_sm[16] = { 0 };
+  static std::atomic<int> per_sm[16] = {}; // per device, 0 = not known yet; two threads may both find it, the same way
   int dev = 0;
   B200_CUDA_TRY(cudaGetDevice(&dev));
-  if(!per_sm[dev & 15])
+  int resident = per_sm[dev & 15].load(std::memory_order_acquire);
+  if(!resident)
   {
     B200_CUDA_TRY(cudaFuncSetAttribute(amaze_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)HALF));
     int n = 0;
     B200_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, amaze_tiles_kernel, NT, HALF));
-    per_sm[dev & 15] = n < 1 ? 1 : n;
+    resident = n < 1 ? 1 : n;
+    per_sm[dev & 15].store(resident, std::memory_order_release);
   }
-  int grid = per_sm[dev & 15] * sm_count();
+  int grid = resident * sm_count();
   if(grid > a.ntiles) grid = a.ntiles;
   void *scr = nullptr;
   int rc = scratch(SLOT_TMP2, (size_t)grid * SCRATCH_STRIDE, &scr);

@@ -17,6 +17,8 @@
 // Algorithmic bytes: 20 B/px (SURVEY.md 8d).
 #ifndef B200_KERNELS_ON_CPU // tests/emul compiles the stages of this file with g++ to check them against the oracle without a GPU
 #include "runtime.h"
+#include <atomic>
+#include <mutex>
 #endif
 #include <math.h>
 #include <string.h>
@@ -451,27 +453,40 @@ int lmmse_demosaic_dev(const float *d_in, float *d_out, int width, int height, u
       if(b200_fc(r, c, filters) != b200_fc(r & 1, c, filters)) return fail(B200_ERR_UNSUPPORTED, "LMMSE: filters 0x%08x is not a 2x2 Bayer pattern", filters);
   int dev = 0;
   B200_CUDA_TRY(cudaGetDevice(&dev));
-  static float *d_tables[16] = { nullptr }; // per device: gamma_in, gamma_out
-  if(!d_tables[dev & 15])
+  // per device: gamma_in, gamma_out.  Made once under the lock and published only when uploaded, so no thread launches on
+  // tables still being filled.
+  static std::atomic<float *> d_tables[16] = {};
+  static std::mutex tables_mu;
+  float *tables = d_tables[dev & 15].load(std::memory_order_acquire);
+  if(!tables)
   {
-    float *h = (float *)malloc(2 * 65536 * sizeof(float));
-    if(!h) return fail(B200_ERR_ARG, "LMMSE: out of host memory");
-    lm_gamma_tables(h, h + 65536);
-    cudaError_t e = cudaMalloc(&d_tables[dev & 15], 2 * 65536 * sizeof(float));
-    if(e == cudaSuccess) e = cudaMemcpy(d_tables[dev & 15], h, 2 * 65536 * sizeof(float), cudaMemcpyHostToDevice);
-    free(h);
-    if(e != cudaSuccess)
+    std::lock_guard<std::mutex> lock(tables_mu);
+    tables = d_tables[dev & 15].load(std::memory_order_acquire); // another thread may have made them meanwhile
+    if(!tables)
     {
-      d_tables[dev & 15] = nullptr;
-      return fail(B200_ERR_CUDA, "LMMSE: gamma tables: %s", cudaGetErrorString(e));
+      float *h = (float *)malloc(2 * 65536 * sizeof(float));
+      if(!h) return fail(B200_ERR_ARG, "LMMSE: out of host memory");
+      lm_gamma_tables(h, h + 65536);
+      float *d = nullptr;
+      cudaError_t e = cudaMalloc(&d, 2 * 65536 * sizeof(float));
+      if(e == cudaSuccess) e = cudaMemcpyAsync(d, h, 2 * 65536 * sizeof(float), cudaMemcpyHostToDevice, stream);
+      if(e == cudaSuccess) e = cudaStreamSynchronize(stream); // complete before another thread's stream may read them
+      free(h);
+      if(e != cudaSuccess)
+      {
+        if(d) cudaFree(d);
+        return fail(B200_ERR_CUDA, "LMMSE: gamma tables: %s", cudaGetErrorString(e));
+      }
+      tables = d;
+      d_tables[dev & 15].store(tables, std::memory_order_release);
     }
   }
   lm_args_t a;
   lm_plan(a, width, height, filters, mode, processed_maximum);
   a.in = d_in;
   a.out = (float4 *)d_out;
-  a.gamma_in = d_tables[dev & 15];
-  a.gamma_out = d_tables[dev & 15] + 65536;
+  a.gamma_in = tables;
+  a.gamma_out = tables + 65536;
   int grid = sm_count();
   if(grid > a.nv * a.nh) grid = a.nv * a.nh;
   void *scr = nullptr;

@@ -26,6 +26,7 @@
 #include <float.h>
 #include <string.h>
 #include <vector>
+#include <atomic>
 
 namespace
 {
@@ -587,22 +588,50 @@ int mk_build_classes(mk_args_t &a, std::vector<short> &maps)
 #ifndef B200_KERNELS_ON_CPU
 struct mk_plan_t
 { // what depends on the geometry only: built once per (frame size, origin, pattern), kept on the device
-  int width = 0, height = 0, rx = 0, ry = 0, dev = -1, passes = 0;
+  int width = 0, height = 0, rx = 0, ry = 0, dev = -1, passes = 0; // dev < 0: matches no call
   uint8_t xtrans[36] = { 0 };
   mk_args_t a;
   short *d_start = nullptr;
+  cudaEvent_t used = nullptr; // recorded after every launch that reads d_start, on the stream it went to
+
+  cudaError_t release()
+  { // waits for the last launch that read the maps, on whichever stream it went to, then frees them
+    cudaError_t e = used ? cudaEventSynchronize(used) : cudaSuccess;
+    if(d_start && e == cudaSuccess) e = cudaFree(d_start);
+    if(used) cudaEventDestroy(used);
+    *this = mk_plan_t();
+    return e;
+  }
 };
-mk_plan_t g_plan[2];
+struct mk_plans_t
+{ // per calling thread, as the device scratch is (runtime.cu): two geometries (the preview and the full pipe), replaced in turn
+  mk_plan_t plan[2];
+  int next = 0;
+  ~mk_plans_t()
+  {
+    if(!b200::runtime_alive()) return;
+    int cur = 0;
+    cudaGetDevice(&cur);
+    for(auto &p : plan)
+      if(p.d_start || p.used)
+      {
+        cudaSetDevice(p.dev < 0 ? cur : p.dev);
+        p.release();
+      }
+    cudaSetDevice(cur);
+  }
+};
+thread_local mk_plans_t tls_plans;
 
 template <int PASSES> int mk_launch(mk_args_t &a, int dev, cudaStream_t stream)
 {
   using geo = mk_geo<PASSES>;
-  static bool attr_set[16] = { false };
+  static std::atomic<bool> attr_set[16] = {}; // per device; setting it twice from two threads is harmless
   const int smem = geo::NDIR * NPX;
-  if(!attr_set[dev & 15])
+  if(!attr_set[dev & 15].load(std::memory_order_acquire))
   {
     B200_CUDA_TRY(cudaFuncSetAttribute(markesteijn_tiles_kernel<PASSES>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    attr_set[dev & 15] = true;
+    attr_set[dev & 15].store(true, std::memory_order_release);
   }
   int grid = b200::sm_count();
   if(grid > a.ntiles) grid = a.ntiles;
@@ -614,7 +643,6 @@ template <int PASSES> int mk_launch(mk_args_t &a, int dev, cudaStream_t stream)
   B200_CUDA_TRY(cudaGetLastError());
   return B200_OK;
 }
-int g_plan_next = 0;
 #endif
 } // namespace
 
@@ -635,18 +663,15 @@ int markesteijn_demosaic_dev(const float *d_in, float *d_out, int width, int hei
   int dev = 0;
   B200_CUDA_TRY(cudaGetDevice(&dev));
   mk_plan_t *plan = nullptr;
-  for(auto &q : g_plan)
+  for(auto &q : tls_plans.plan)
     if(q.d_start && q.dev == dev && q.passes == passes && q.width == width && q.height == height && q.rx == x0 && q.ry == y0 && !memcmp(q.xtrans, xtrans, 36)) plan = &q;
   if(!plan)
   {
-    plan = &g_plan[g_plan_next];
-    g_plan_next ^= 1;
-    if(plan->d_start)
-    {
-      B200_CUDA_TRY(cudaStreamSynchronize(stream));
-      B200_CUDA_TRY(cudaFree(plan->d_start));
-      plan->d_start = nullptr;
-    }
+    plan = &tls_plans.plan[tls_plans.next];
+    tls_plans.next ^= 1;
+    // a frame queued on another of this thread's streams may still read the maps being replaced: release() waits for it
+    B200_CUDA_TRY(plan->release());
+    B200_CUDA_TRY(cudaEventCreateWithFlags(&plan->used, cudaEventDisableTiming));
     mk_args_t &a = plan->a;
     memset(&a, 0, sizeof(a));
     a.width = width;
@@ -666,15 +691,16 @@ int markesteijn_demosaic_dev(const float *d_in, float *d_out, int width, int hei
     plan->height = height;
     plan->rx = x0;
     plan->ry = y0;
-    plan->dev = dev;
     plan->passes = passes;
     memcpy(plan->xtrans, xtrans, 36);
+    plan->dev = dev; // complete: from here on the plan matches
   }
   mk_args_t a = plan->a;
   a.in = d_in;
   a.out = (float4 *)d_out;
   const int rc = passes == 1 ? mk_launch<1>(a, dev, stream) : mk_launch<3>(a, dev, stream);
   if(rc) return rc;
+  B200_CUDA_TRY(cudaEventRecord(plan->used, stream));
   return B200_OK;
 }
 } // namespace b200

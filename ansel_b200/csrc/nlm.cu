@@ -24,6 +24,7 @@
 // Not HBM bound by construction (SURVEY.md 8d: ~9 kflop/px at K=7); reported against FP32 issue.
 #ifndef B200_KERNELS_ON_CPU // tests/emul compiles the group kernel's phases with g++ to check them against the oracle without a GPU
 #include "runtime.h"
+#include <atomic>
 #include <math_constants.h>
 #endif
 #include <math.h>
@@ -888,24 +889,26 @@ int nlmeans_denoise_dev(const float *d_in, float *d_out, int width, int height, 
   a.plane_e = a.rows_e * SW;
   a.cols_w = a.chk_w + 2 * radius + 2;
   a.sstride_w = a.cols_w | 1;
-  static bool attr_set[16] = { false };
-  static int smem_optin[16] = { 0 };
+  // per device, 0 until the kernels' shared-memory attributes are set: one atomic, so no thread sees "set" without the
+  // limit.  Two threads may both set them, to the same values.
+  static std::atomic<int> smem_optin[16] = {};
   int dev = 0;
   B200_CUDA_TRY(cudaGetDevice(&dev));
-  if(!attr_set[dev & 15])
+  int optin = smem_optin[dev & 15].load(std::memory_order_acquire);
+  if(!optin)
   {
     const int smem_max = 2 * (3 * (MAX_CH + 2 * MAX_RADIUS + 1) * SW + MAX_CH * SSTRIDE) * (int)sizeof(float);
     B200_CUDA_TRY(cudaFuncSetAttribute(nlm_chunks_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
-    B200_CUDA_TRY(cudaDeviceGetAttribute(&smem_optin[dev & 15], cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-    B200_CUDA_TRY(cudaFuncSetAttribute(nlm_chunks_win_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin[dev & 15]));
-    attr_set[dev & 15] = true;
+    B200_CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    B200_CUDA_TRY(cudaFuncSetAttribute(nlm_chunks_win_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
+    smem_optin[dev & 15].store(optin, std::memory_order_release);
   }
   // The group kernel (nlm_group.cuh) wherever the pixels a chunk reads for every patch, plus at least two planes of
   // column sums, fit the shared memory of an SM: every module default does (K = 7 with P <= 4 and no scattering).
   if(!getenv("B200_NLM_CHUNKS") && !getenv("B200_NLM_WINDOW"))
   {
     int launched = 0;
-    if((rc = launch_group(a, h_shift_max, smem_optin[dev & 15], n_ct * a.n_cl, stream, &launched))) return rc;
+    if((rc = launch_group(a, h_shift_max, optin, n_ct * a.n_cl, stream, &launched))) return rc;
     if(launched) return B200_OK;
   }
   const long long win_bytes = 2LL * a.rows_e * a.cols_w * 16 + 2LL * a.chk_h * a.sstride_w * 4;
@@ -913,7 +916,7 @@ int nlmeans_denoise_dev(const float *d_in, float *d_out, int width, int height, 
   // moves all global traffic into one cp.async fill per patch but spends twice the instructions on index
   // arithmetic in its parallel phases).  The window kernel stays selectable for that follow-up work.
   const bool use_window = getenv("B200_NLM_WINDOW") != nullptr;
-  if(use_window && win_bytes <= smem_optin[dev & 15])
+  if(use_window && win_bytes <= optin)
     nlm_chunks_win_kernel<<<(unsigned)(n_ct * a.n_cl), WNT, (size_t)win_bytes, stream>>>(a);
   else
   {

@@ -30,6 +30,7 @@
 // HBM traffic per tile: 112*112*4 B read (1.42x over-read from the 18-px overlap, served by L2),
 // 94*94*16 B written.  Algorithmic bytes: 20 B/px (SURVEY.md 8d).
 #include "runtime.h"
+#include <atomic>
 
 namespace
 {
@@ -515,14 +516,14 @@ int rcd_demosaic_dev(const float *d_in, float *d_out, int width, int height, uin
   if(!standard_bayer(filters))
     return fail(B200_ERR_UNSUPPORTED, "RCD: filters 0x%08x is not a 2x2 Bayer pattern", filters);
 
-  static bool attr_set[16] = { false };
+  static std::atomic<bool> attr_set[16] = {}; // per device; setting it twice from two threads is harmless
   int dev = 0;
   B200_CUDA_TRY(cudaGetDevice(&dev));
   const int smem_bytes = SMEM_FLOATS * (int)sizeof(float);
-  if(!attr_set[dev & 15])
+  if(!attr_set[dev & 15].load(std::memory_order_acquire))
   {
     B200_CUDA_TRY(cudaFuncSetAttribute(rcd_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
-    attr_set[dev & 15] = true;
+    attr_set[dev & 15].store(true, std::memory_order_release);
   }
 
   const long long ring_px = 2LL * EDGE * width + 2LL * EDGE * (height - 2 * EDGE);

@@ -252,23 +252,33 @@ struct timed_pair
   cudaEvent_t e0, e1;
 };
 std::vector<timed_pair> g_timed[TIMED_COUNT];
+unsigned g_timed_gen = 0; // bumped by every b200_kernel_timing(): the indices handed out before it are void
 const char *const g_timed_names[TIMED_COUNT] = { "nlm_kernel", "rcd_tiles_kernel" } /* nlm_kernel: whichever non-local-means kernel the launcher picked (nlm_pipe_kernel for the bench frame) */;
 } // namespace
 bool timing_enabled() { return g_timing.load(std::memory_order_relaxed); }
-void timing_mark(int which, bool end, cudaStream_t stream)
+int timing_start(int which, cudaStream_t stream, unsigned *generation)
 {
   std::lock_guard<std::mutex> lock(g_timing_mu);
-  if(which < 0 || which >= TIMED_COUNT) return;
-  if(!end)
+  if(which < 0 || which >= TIMED_COUNT || !g_timing.load()) return -1;
+  timed_pair p = { nullptr, nullptr };
+  if(cudaEventCreate(&p.e0) != cudaSuccess) return -1;
+  if(cudaEventCreate(&p.e1) != cudaSuccess)
   {
-    timed_pair p = { nullptr, nullptr };
-    if(cudaEventCreate(&p.e0) != cudaSuccess || cudaEventCreate(&p.e1) != cudaSuccess) return;
-    cudaEventRecord(p.e0, stream);
-    g_timed[which].push_back(p);
+    cudaEventDestroy(p.e0);
+    return -1;
   }
-  else if(!g_timed[which].empty())
-    cudaEventRecord(g_timed[which].back().e1, stream);
+  cudaEventRecord(p.e0, stream);
+  g_timed[which].push_back(p);
+  *generation = g_timed_gen;
+  return (int)g_timed[which].size() - 1;
 }
+void timing_end(int which, int index, unsigned generation, cudaStream_t stream)
+{
+  std::lock_guard<std::mutex> lock(g_timing_mu);
+  if(which < 0 || which >= TIMED_COUNT || generation != g_timed_gen || index < 0 || index >= (int)g_timed[which].size()) return;
+  cudaEventRecord(g_timed[which][index].e1, stream);
+}
+bool runtime_alive() { return g_alive.load(); }
 } // namespace b200
 
 // ---- exported C ABI ---------------------------------------------------------------------
@@ -286,6 +296,7 @@ extern "C" int b200_kernel_timing(int enable)
     }
     v.clear();
   }
+  g_timed_gen++;
   g_timing.store(enable != 0);
   return B200_OK;
 }

@@ -61,21 +61,28 @@ enum
   TIMED_COUNT = 2
 };
 bool timing_enabled();
-void timing_mark(int which, bool end, cudaStream_t stream);
+// Records the start event of a new pair and returns its index (-1: not recorded); `generation` identifies the recording
+// the pair belongs to, so an end mark after a b200_kernel_timing() clear records nothing.
+int timing_start(int which, cudaStream_t stream, unsigned *generation);
+void timing_end(int which, int index, unsigned generation, cudaStream_t stream);
 struct timed_launch
-{ // brackets the statement(s) between construction and destruction
-  int which;
+{ // brackets the statement(s) between construction and destruction; the end goes into this launch's own pair, whatever
+  // other threads time meanwhile
+  int which, index;
+  unsigned generation;
   cudaStream_t stream;
-  bool on;
-  timed_launch(int w, cudaStream_t s) : which(w), stream(s), on(timing_enabled())
+  timed_launch(int w, cudaStream_t s) : which(w), index(-1), generation(0), stream(s)
   {
-    if(on) timing_mark(which, false, stream);
+    if(timing_enabled()) index = timing_start(which, stream, &generation);
   }
   ~timed_launch()
   {
-    if(on) timing_mark(which, true, stream);
+    if(index >= 0) timing_end(which, index, generation, stream);
   }
 };
+
+// false before b200_init() and after b200_shutdown(): the CUDA context may be gone, per-thread state is not freed then
+bool runtime_alive();
 
 // Device copy of three tone curves (3 * B200_LUT_SAMPLES floats), cached per device by `identity` and `side`
 // (0 = decoding / source, 1 = encoding / target); identity 0 = upload every time.  color.cu.

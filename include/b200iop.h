@@ -14,8 +14,11 @@
  * a process_cl() adapter returns `rc == 0` because that slot means TRUE = success
  * (develop/pixelpipe_gpu.c:358).
  *
- * Threading: entry points are re-entrant; up to four pipes may run the same module concurrently
- * (doc/reorganisation.md:77-81).  Device scratch is per calling thread and per device.
+ * Threading: entry points are re-entrant.  Any number of threads may run the same module at once, each on its own
+ * stream(s), as the reference's pipes do (doc/reorganisation.md:77-81): the darkroom's preview and full pipes, the frames
+ * of a batch export.  Device scratch and the geometry plans of the demosaicers are per calling thread and per device.
+ * One thread that drives several streams must order the modules that share its scratch, as b200_pixelpipe_submit does
+ * with its `compute_done` events.
  * There is no CPU fallback anywhere in this library: without a CUDA device calls fail.
  */
 #ifndef B200IOP_H
@@ -111,9 +114,10 @@ void b200_shutdown(void);
 int b200_device_count(void);
 /* thread-local, never NULL */
 const char *b200_last_error(void);
-/* Launch timing of the two headline kernels, for benchmarks: while enabled, every launch of `nlm_group_kernel` (non-local
- * means, nlm_group.cuh) and `rcd_tiles_kernel` (RCD demosaic, rcd.cu) is bracketed by a pair of CUDA events on the stream it
- * is launched on.  b200_kernel_timing(1) clears what was recorded and starts, (0) clears and stops;
+/* Launch timing of the two headline kernels, for benchmarks: while enabled, every launch of `nlm_kernel` (whichever
+ * non-local-means kernel the launcher picked: nlm.cu, nlm_group.cuh) and `rcd_tiles_kernel` (RCD demosaic, rcd.cu) is
+ * bracketed by its own pair of CUDA events on the stream it is launched on, from any thread.
+ * b200_kernel_timing(1) clears what was recorded and starts, (0) clears and stops;
  * b200_kernel_timing_read() waits for the recorded launches of one kernel and returns their summed duration and count.
  * No counterpart in the reference (its OpenCL path profiles through dt_opencl_events_*, src/common/opencl.c). */
 int b200_kernel_timing(int enable);
